@@ -47,7 +47,12 @@ def parse():
     ap.add_argument("--workload", default=os.environ.get("CCO_BENCH_WORKLOAD", "C3"))
     ap.add_argument("--cpu-sample", default="auto", help="oracle sample: 'full', 'none' or a user fraction like 0.1")
     ap.add_argument("--seed", type=int, default=42)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the indicators of the last timed steps to DIR/<name>.npy (float64; see dump_outputs)")
+    a = ap.parse_args()
+    if a.dump_outputs is not None and a.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
+    return a
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -95,6 +100,37 @@ def algorithmic_bytes(st, i: int, n_items_a: int) -> float:
     nnz_a = st.nnz_downsampled[0]
     return (4.0 * nnz_a + 8.0 * (n_items_a + 1) + 8.0 * nnz_a + 4.0 * st.products[i] + 4.0 * st.distinct_cells[i]
             + 4.0 * n_items_a + 12.0 * st.out_nnz[i])
+
+
+DUMP_BYTES = 56 << 20   # --dump-outputs stays under 64 MB: larger models are cut to a sample of their rows
+
+
+def dump_outputs(out_dir: str, e2e, resident, top_k: int):
+    """--dump-outputs: what the last timed steps returned, as float64 .npy files, so that two builds can be compared output
+    for output.  e2e: the result of cco_train, [(row_begin, row_end, n_cols, row_ptr, col_idx, llr, count)] per indicator
+    (the end-to-end leg asks for no counts); resident: the resident step's result, of which only row_ptr reaches the host.
+      rows.npy                           primary-item rows written: every row, or a fixed seeded sample when the model is
+                                         larger than DUMP_BYTES (the same rows for every indicator)
+      indicator<i>_row_len.npy           kept cells per written row (cco_train)
+      indicator<i>_col_idx.npy           their column ids, row after row, in result order (cco_train)
+      indicator<i>_llr.npy               their LLR values (cco_train)
+      indicator<i>_resident_row_len.npy  kept cells per written row (resident step)"""
+    n_rows = len(e2e[0][3]) - 1
+    per_row = 8 + len(e2e) * (8 + 8 + 16 * top_k)      # a row holds at most top_k cells
+    n = min(n_rows, DUMP_BYTES // per_row)
+    rows = np.arange(n_rows) if n == n_rows else np.sort(np.random.default_rng(0).choice(n_rows, n, replace=False))
+    arrays = {"rows": rows}
+    for i, (r, d) in enumerate(zip(e2e, resident)):
+        rp = r[3]
+        start, lens = rp[rows], rp[rows + 1] - rp[rows]
+        take = np.repeat(start - np.cumsum(lens) + lens, lens) + np.arange(int(lens.sum()))
+        arrays[f"indicator{i}_row_len"] = lens
+        arrays[f"indicator{i}_col_idx"] = r[4][take]
+        arrays[f"indicator{i}_llr"] = r[5][take]
+        arrays[f"indicator{i}_resident_row_len"] = d[3][rows + 1] - d[3][rows]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 def ncu_traffic(workload: str):
@@ -305,6 +341,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device -- this framework has no CPU fallback")
+    if args.dump_outputs is not None and world > 1:
+        raise SystemExit("bench.py: --dump-outputs writes one process's model: run it on one GPU")
     torch.cuda.set_device(local_rank)
     uid = None
     if world > 1:
@@ -361,7 +399,7 @@ def main():
     rows_ms, launches = 0.0, 0
     alg_bytes = 0.0
     for _ in range(args.steps):
-        ctx.train_dataset(ds, w.params, args.seed, flags | N.FLAG_RESULT_ON_DEVICE, copy_arrays=False)
+        resident_last = ctx.train_dataset(ds, w.params, args.seed, flags | N.FLAG_RESULT_ON_DEVICE, copy_arrays=False)
         st = ctx.last_stats
         rows_ms += sum(st.ms_indicator)
         launches += st.n_kernel_launches
@@ -381,7 +419,7 @@ def main():
     # co-occurrence count k11 is a by-product nothing downstream reads, so the end-to-end leg does not copy it back
     flags_e2e = flags | N.FLAG_RESULT_NO_COUNT
 
-    def e2e_step():
+    def e2e_step(keep: bool = False):
         res, h = ctx.train_csr(pinned, w.params, args.seed, flags_e2e, keep=True)
         nbytes = sum(r[3].nbytes + r[4].nbytes + r[5].nbytes + r[6].nbytes for r in res)
         if shm is not None:
@@ -392,18 +430,23 @@ def main():
                 assert sum(sl[0][1] - sl[0][0] for sl in model) == n_items_a
                 assert all(int(sl[i][2][-1]) == len(sl[i][3]) for sl in model for i in range(w.n_types))
             dist.barrier()          # the slices are read in place: nobody frees before rank 0 is done
+        if keep:                    # --dump-outputs reads the last step's arrays after the timed region
+            return nbytes, res, h
         ctx.free_result(h)
-        return nbytes
+        return nbytes, None, None
 
     for _ in range(args.warmup):
         e2e_step()
     barrier()
     t0 = time.perf_counter()
-    d2h_bytes = 0
-    for _ in range(args.steps):
-        d2h_bytes = e2e_step()
+    d2h_bytes, last_res, last_h = 0, None, None
+    for s in range(args.steps):
+        d2h_bytes, last_res, last_h = e2e_step(keep=args.dump_outputs is not None and s == args.steps - 1)
     torch.cuda.synchronize()
     wall_e2e = (time.perf_counter() - t0) * 1e3
+    if last_h is not None:
+        dump_outputs(args.dump_outputs, last_res, resident_last, max(p[1] for p in w.params))
+        ctx.free_result(last_h)
     barrier()
     ms_e2e = max_over_ranks(wall_e2e) / args.steps
     e2e_value = w.n_events / (ms_e2e * 1e-3)

@@ -6,6 +6,7 @@ import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 from conftest import ROOT
 
@@ -64,3 +65,51 @@ def test_algorithmic_bytes_formula():
         out_nnz = [3_000, 4_000]
     # SURVEY.md 8(d): 4 nnz(A') + 8 (I_A+1) + 8 nnz(A') + 4 P + 4 C + 4 I_A + 12 out
     assert bench.algorithmic_bytes(St, 1, 100) == 4 * 1000 + 8 * 101 + 8 * 1000 + 4 * 70_000 + 4 * 60_000 + 4 * 100 + 12 * 4_000
+
+
+def _read_dump(d):
+    return {f[:-4]: np.load(os.path.join(d, f)) for f in sorted(os.listdir(d))}
+
+
+def test_dump_outputs_samples_whole_rows_under_the_size_limit(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    rng = np.random.default_rng(1)
+    n_rows, k = 20_000, 50
+    model = []
+    for _ in range(3):
+        rp = np.concatenate([[0], np.cumsum(rng.integers(0, k + 1, n_rows))]).astype(np.int64)
+        model.append((0, n_rows, n_rows, rp, rng.integers(0, n_rows, rp[-1]).astype(np.int32), rng.random(rp[-1]),
+                      np.zeros(0, np.int32)))
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), model, model, k)
+    a, b = _read_dump(tmp_path / "a"), _read_dump(tmp_path / "b")
+    assert a.keys() == b.keys() and all(np.array_equal(a[n], b[n]) for n in a)          # a fixed sample
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= (1 << 20) + 4096
+    assert all(x.dtype == np.float64 for x in a.values())
+    rows = a["rows"].astype(np.int64)
+    assert 0 < len(rows) < n_rows and (np.diff(rows) > 0).all()
+    for i, (_, _, _, rp, ci, ll, _) in enumerate(model):
+        want = np.concatenate([np.arange(rp[r], rp[r + 1]) for r in rows])
+        assert np.array_equal(a[f"indicator{i}_row_len"], np.diff(rp)[rows])
+        assert np.array_equal(a[f"indicator{i}_resident_row_len"], np.diff(rp)[rows])
+        assert np.array_equal(a[f"indicator{i}_col_idx"], ci[want]) and np.array_equal(a[f"indicator{i}_llr"], ll[want])
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_repeat_and_match_the_oracle(orc, tmp_path):
+    import synth
+    for d in ("a", "b"):
+        subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "tiny", "--steps", "2", "--warmup", "1",
+                        "--cpu-sample", "none", "--dump-outputs", str(tmp_path / d)], capture_output=True, text=True, check=True)
+    a, b = _read_dump(tmp_path / "a"), _read_dump(tmp_path / "b")
+    assert a.keys() == b.keys() and all(np.array_equal(a[n], b[n]) for n in a)
+    w = synth.make("tiny")
+    ref = orc.train([orc.Csr(*m) for m in w.mats], [orc.Params(*p) for p in w.params], 42)
+    assert np.array_equal(a["rows"], np.arange(w.n_items))                                # tiny: every row is written
+    for i, r in enumerate(ref):
+        assert np.array_equal(a[f"indicator{i}_row_len"], np.diff(r.row_ptr))
+        assert np.array_equal(a[f"indicator{i}_resident_row_len"], np.diff(r.row_ptr))
+        assert np.array_equal(a[f"indicator{i}_col_idx"], r.col_idx)
+        assert np.allclose(a[f"indicator{i}_llr"], r.llr, rtol=1e-6, atol=0)

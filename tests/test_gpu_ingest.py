@@ -46,10 +46,11 @@ def test_ingest_edge_cases(orc, ctx):
 
 
 @pytest.mark.parametrize("name", ["tiny", "small", "C3-tenth"])
-def test_device_generator_matches_numpy_twin(ctx, name):
+def test_device_generator_matches_numpy_twin(ctx, name, monkeypatch):
     """cco_synth_ingest (events generated and ingested in HBM) and synth.py's numpy path give the same matrices bit for bit:
     same counter-based stream, same Preparator semantics (user dictionary from the primary events, dedup)."""
     import synth
+    monkeypatch.setenv("CCO_SYNTH_CACHE", "0")     # a cached file from an earlier run is not the numpy path under test
     host = synth.make(name)
     dev = synth.make(name, ctx=ctx)
     assert host.n_users == dev.n_users

@@ -3,7 +3,7 @@
   level-1 strong cells with colB > c1* cannot be in the top-k (LLR strictly decreasing in colB) -> never evaluated;
   every other cell is evaluated as today.  Exact."""
 import sys
-sys.path.insert(0, __import__('os').path.dirname(__import__('os').path.dirname(__import__('os').path.dirname(__import__('os').path.abspath(__file__))))); sys.path.insert(0, '/tmp/proto')
+sys.path.insert(0, __import__('os').path.dirname(__import__('os').path.dirname(__import__('os').path.dirname(__import__('os').path.abspath(__file__)))))
 from select_model import llr, brute, random_row
 import random
 
