@@ -680,6 +680,15 @@ static int launch_rows(cco_ctx *c, const RowArgs &a, BinCfg &cfg, cudaStream_t s
   return set_error(CCO_E_INVALID_ARG, "internal: bad bin config");
 }
 
+// Candidate-buffer invariant of k_rows (checked by cfg_ok before any launch):
+//   top_k <= keep_max <= cbuf - group   and   final_max <= cbuf,   caux >= max(keep_max, final_max) for CTA groups.
+// A round appends at most `group` candidates to a buffer that holds at most prune_limit = cbuf - group of them (no
+// prune) or keep_max (after a prune), so it never writes past cbuf; the CTA-path select compacts up to keep_max (or
+// final_max) survivors into aux.  keep_max is capped at cbuf - group: without the cap, final_max = next_pow2(top_k)
+// exceeds the prune limit in some CTA configurations (group 128: top_k 257-384, 513-896, 1025-1920; group 256: 513-768,
+// 1025-1792; group 512: 1025-1536; e.g. top_k 300, group 128: cbuf 512, limit 384, keep_max 512), a prune may stop
+// with nearly every candidate kept, and the next round overflows tk into aux.  The cap changes keep_max in those
+// configurations only; caux (max(keep_max, final_max)), hence the shared-memory layout, is the same as before everywhere.
 static BinCfg make_cfg(cco_ctx *c, int group, int want_slots, int top_k, int n_cols_b) {
   BinCfg f;
   const int groups = group == 32 ? 2 : 1;
@@ -687,8 +696,8 @@ static BinCfg make_cfg(cco_ctx *c, int group, int want_slots, int top_k, int n_c
   f.final_max = next_pow2(top_k);
   f.cbuf = next_pow2(top_k + std::max(group, 128) + (group == 32 ? 64 : 0));
   if (group == 32 && top_k + 32 <= 96) f.cbuf = 128;  // small top_k: a 128-entry buffer doubles the warps per SM (-4 % at C3)
-  f.keep_max = std::max(f.final_max, (f.cbuf - group) / 2);
-  f.caux = group == 32 ? 0 : f.keep_max;
+  f.keep_max = std::min(std::max(f.final_max, (f.cbuf - group) / 2), f.cbuf - group);
+  f.caux = group == 32 ? 0 : std::max(f.keep_max, f.final_max);
   // candidates, x12/x11 tables, ctrl, radix-select histogram (aliased by the level-1 cut bins), queues
   size_t fixed = (size_t)(f.cbuf + f.caux) * 16 + 2 * 256 + 512 + 1024 + (size_t)(group / 32) * 256;
   size_t avail = (c->smem_optin - 1024) / groups;  // slack for static shared memory
@@ -700,6 +709,11 @@ static BinCfg make_cfg(cco_ctx *c, int group, int want_slots, int top_k, int n_c
   f.smem = f.region * groups;
   f.ctas_per_sm = 1;
   return f;
+}
+
+static bool cfg_ok(const BinCfg &f, int top_k, size_t smem_optin) {
+  return top_k <= f.keep_max && f.keep_max <= f.cbuf - f.group && f.final_max <= f.cbuf &&
+         (f.group == 32 || f.caux >= std::max(f.keep_max, f.final_max)) && f.slots > 0 && f.smem <= smem_optin;
 }
 
 // ---- one indicator = rows [lo, hi) of A'^T B' on this rank ---------------------------------------------------------------
@@ -788,7 +802,13 @@ static int enqueue_indicator(cco_ctx *c, Arena &ar, const uint32_t *at_ptr, cons
   }
   const int kBins = (int)spec.size();
   std::vector<BinCfg> cfgs(kBins);
-  for (int b = 0; b < kBins; ++b) cfgs[b] = make_cfg(c, spec[b].group, spec[b].slots, k_eff, n_cols_b);
+  for (int b = 0; b < kBins; ++b) {
+    cfgs[b] = make_cfg(c, spec[b].group, spec[b].slots, k_eff, n_cols_b);
+    if (!cfg_ok(cfgs[b], k_eff, c->smem_optin))
+      return set_error(CCO_E_INVALID_ARG, "internal: row-kernel bin %d (group %d, top_k %d) violates the candidate-buffer "
+                       "invariant: cbuf %d, keep_max %d, final_max %d, caux %d", b, spec[b].group, k_eff, cfgs[b].cbuf,
+                       cfgs[b].keep_max, cfgs[b].final_max, cfgs[b].caux);
+  }
   BinCfg &cfgL = cfgs[1];
   // packed word: key bits must leave room for the largest possible count
   int key_bits = 1;
