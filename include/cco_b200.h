@@ -95,7 +95,10 @@ enum {
    * drops the LLR values, nothing reads k11): NO_COUNT skips the count array (cco_result_matrix returns NULL for it),
    * NO_LLR skips the LLR array too -- 80 instead of 321 MB come back per train at C3. */
   CCO_FLAG_RESULT_NO_COUNT = 16,
-  CCO_FLAG_RESULT_NO_LLR = 32
+  CCO_FLAG_RESULT_NO_LLR = 32,
+  /* tests only, not for production (cco_ingest_strings): the id hash keeps 2 bits, so nearly every pair of distinct ids
+   * collides and the exact byte-comparison pass does the grouping.  The output is the same, only slower. */
+  CCO_FLAG_INGEST_SHORT_HASH = 64
 };
 
 /*
@@ -291,6 +294,30 @@ typedef struct {
 } cco_dictionary_t;
 int cco_format_es_bulk(cco_ctx_t *ctx, const cco_result_t *res, int32_t n_names, const char *const *names,
                        const cco_dictionary_t *row_ids, const cco_dictionary_t *col_ids, char **out_bytes, int64_t *out_len);
+
+/*
+ * Preparator.prepare from raw id strings (src/main/scala/Preparator.scala:111-126, 170-190), on the device.  Event type t
+ * is two columns of strings: the user and the item id of event e are user.bytes / item.bytes [offsets[e] .. offsets[e + 1]).
+ * Two ids are equal iff their bytes are equal (no normalisation; NUL, the empty id and non-ASCII bytes are ordinary ids).
+ *  - user_dict: users of type 0 with at least min_events_per_user type-0 events (duplicates count; 0 or 1 = any), in order
+ *    of first appearance among the type-0 events.  Users seen only in other types are dropped.
+ *  - item_dicts[t]: the items of the type-t events whose user is in user_dict, in order of first appearance among those
+ *    events.  Every type has its own id space.
+ *  - *out: the same resident dataset cco_ingest builds from the same tokens (n_rows = user_dict.n for every type, columns
+ *    ascending within a row, duplicates collapsed), ready for cco_train_dataset.
+ * Every offsets / bytes pointer written into user_dict and item_dicts is pinned memory owned by the context: release each
+ * with cco_host_free.  On error nothing is written and nothing is kept.
+ * Errors: CCO_E_INVALID_ARG for null pointers, n_types < 1, user.n != item.n, n >= 2^32 events in a type, offsets[0] != 0
+ * or decreasing offsets (all checked before the id bytes are read); CCO_E_UNSUPPORTED for a group context and for more
+ * than 2^31 - 2 distinct type-0 users or distinct items in one item dictionary.
+ */
+typedef struct {
+  cco_dictionary_t user; /* user.n == item.n == number of events */
+  cco_dictionary_t item;
+} cco_string_events_t;
+int cco_ingest_strings(cco_ctx_t *ctx, int32_t n_types, const cco_string_events_t *events, int32_t min_events_per_user,
+                       uint32_t flags, cco_dictionary_t *user_dict, cco_dictionary_t *item_dicts /* [n_types] */,
+                       cco_dataset_t **out);
 
 /*
  * Next row (SURVEY.md 8f-3): the backfill ranks of PopModel (src/main/scala/PopModel.scala:113-182) as per-item event

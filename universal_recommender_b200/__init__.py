@@ -4,6 +4,7 @@ SimilarityAnalysis) as hand-written sm_100a CUDA behind the C ABI of include/cco
 
 Host-side mirror of the reference interface for this path:
   preparator.prepare                      <- Preparator.prepare           (Preparator.scala:44-87)
+  preparator.prepare_on_device            <- the same from id strings on the B200 (cco_ingest_strings)
   IndexedDataset / BiDictionary           <- Mahout IndexedDataset
   DownsamplableCrossOccurrenceDataset     <- URAlgorithm.scala:336-340
   SimilarityAnalysis.cooccurrencesIDSs / crossOccurrenceDownsampled  <- URAlgorithm.scala:323,343
@@ -12,7 +13,7 @@ Host-side mirror of the reference interface for this path:
 from ._native import (CcoError, CcoInvalidArgument, FLAG_ASSUME_CANONICAL, FLAG_ENTROPY_VARARGS, FLAG_RESULT_NO_COUNT,
                       FLAG_RESULT_NO_LLR, FLAG_ROWRATE_INTDIV, LIB_PATH)
 from .indexed_dataset import BiDictionary, IndexedDataset
-from .preparator import prepare
+from .preparator import prepare, prepare_on_device
 from .similarity_analysis import (CcoContext, DownsamplableCrossOccurrenceDataset, SimilarityAnalysis,
                                   default_context)
 from .ur_algorithm import DefaultURAlgoParams, IndicatorParams, URAlgorithmParams, calc_all
@@ -20,6 +21,6 @@ from .ur_algorithm import DefaultURAlgoParams, IndicatorParams, URAlgorithmParam
 __all__ = [
     "BiDictionary", "CcoContext", "CcoError", "CcoInvalidArgument", "DefaultURAlgoParams",
     "DownsamplableCrossOccurrenceDataset", "IndexedDataset", "IndicatorParams", "SimilarityAnalysis",
-    "URAlgorithmParams", "calc_all", "default_context", "prepare", "FLAG_ASSUME_CANONICAL",
+    "URAlgorithmParams", "calc_all", "default_context", "prepare", "prepare_on_device", "FLAG_ASSUME_CANONICAL",
     "FLAG_ENTROPY_VARARGS", "FLAG_ROWRATE_INTDIV", "FLAG_RESULT_NO_COUNT", "FLAG_RESULT_NO_LLR", "LIB_PATH",
 ]

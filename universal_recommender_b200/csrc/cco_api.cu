@@ -24,6 +24,7 @@
 #include "cco_kernels.cuh"
 #include "cco_sampler.cuh"
 #include "cco_format.cuh"
+#include "cco_strings.cuh"
 
 namespace cco {
 
@@ -2014,6 +2015,323 @@ int cco_synth_ingest(cco_ctx_t *c, int32_t n_types, const cco_synth_type_t *type
   rc = ingest_core(c, src, min_events_per_user, nullptr, nullptr, out);
   drop();
   return rc;
+}
+
+// ---- SURVEY.md 8f-1 from raw id strings (kernels in cco_strings.cuh) ---------------------------------------------------
+// The strings are turned into raw integer ids whose ascending order is the dictionary order (primary users by first
+// appearance, items by first appearance among surviving events); ingest_core then builds the matrices exactly as for
+// cco_ingest.
+namespace cco {
+struct MaxU32 {
+  __device__ __forceinline__ uint32_t operator()(uint32_t a, uint32_t b) const { return a > b ? a : b; }
+};
+static int inclusive_max_u32(cco_ctx *c, Arena &ar, const uint32_t *in, uint32_t *out, unsigned long long n) {
+  size_t tb = 0;
+  CK(cub::DeviceScan::InclusiveScan(nullptr, tb, in, out, MaxU32(), (long long)n, c->stream));
+  void *tmp;
+  CKR(ar.alloc((char **)&tmp, tb));
+  CK(cub::DeviceScan::InclusiveScan(tmp, tb, in, out, MaxU32(), (long long)n, c->stream));
+  ar.release(tmp);
+  return CCO_OK;
+}
+
+// rep[i] = the smallest j < n with bytes(j) == bytes(i), n < 2^32.  Sorting by a 48-bit hash brings equal ids together;
+// each id is compared with the first id of its equal-hash run, and the few that differ from it (hash collisions) are
+// grouped by an exact sort on (hash, bytes, index).  A collision costs time, never a merge of two different ids.
+static int group_ids(cco_ctx *c, Arena &ar, unsigned long long n, const StrCols &cols, bool short_hash, uint32_t *rep) {
+  if (n == 0) return CCO_OK;
+  cudaStream_t s = c->stream;
+  const int bits = short_hash ? 2 : 48;
+  const int G = grid_for((long long)n, 256, c->sm_count);
+  unsigned long long *h, *hs, *n_un;
+  uint32_t *idx, *is, *head, *run, *un;
+  CKR(ar.alloc(&h, n));
+  CKR(ar.alloc(&hs, n));
+  CKR(ar.alloc(&idx, n));
+  CKR(ar.alloc(&is, n));
+  CKR(ar.alloc(&head, n));
+  CKR(ar.alloc(&run, n));
+  CKR(ar.alloc(&un, n));
+  CKR(ar.alloc(&n_un, 1));
+  k_ingest_str_hash<<<G, 256, 0, s>>>(n, cols, (1ULL << bits) - 1, h, idx);
+  size_t tb = 0;
+  CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, h, hs, idx, is, (long long)n, 0, bits, s));
+  void *tmp;
+  CKR(ar.alloc((char **)&tmp, tb));
+  CK(cub::DeviceRadixSort::SortPairs(tmp, tb, h, hs, idx, is, (long long)n, 0, bits, s));
+  ar.release(tmp);
+  k_ingest_str_run_heads<<<G, 256, 0, s>>>(n, hs, head);
+  CKR(inclusive_max_u32(c, ar, head, run, n));
+  CK(cudaMemsetAsync(n_un, 0, 8, s));
+  k_ingest_str_resolve<<<G, 256, 0, s>>>(n, cols, is, run, rep, un, n_un);
+  c->launches += 3;
+  unsigned long long nu = 0;
+  CKR(mail_fetch(c, &nu, n_un, 8));
+  CKR(mail_wait(c));
+  if (nu > 0) {
+    const StrLess less{cols, h};
+    tb = 0;
+    CK(cub::DeviceMergeSort::SortKeys(nullptr, tb, un, (long long)nu, less, s));
+    CKR(ar.alloc((char **)&tmp, tb));
+    CK(cub::DeviceMergeSort::SortKeys(tmp, tb, un, (long long)nu, less, s));
+    ar.release(tmp);
+    const int g = grid_for((long long)nu, 256, c->sm_count);
+    k_ingest_str_class_heads<<<g, 256, 0, s>>>(nu, cols, un, h, head);
+    CKR(inclusive_max_u32(c, ar, head, run, nu));
+    k_ingest_str_class_rep<<<g, 256, 0, s>>>(nu, un, run, rep);
+    c->launches += 2;
+  }
+  for (void *p : {(void *)h, (void *)hs, (void *)idx, (void *)is, (void *)head, (void *)run, (void *)un, (void *)n_un}) ar.release(p);
+  return CCO_OK;
+}
+
+struct DevCol {
+  long long n = 0;
+  long long *off = nullptr;
+  unsigned char *bytes = nullptr;
+};
+static StrCols one_column(const DevCol &d) {
+  StrCols s;
+  s.n_a = d.n;
+  s.off_a = d.off;
+  s.bytes_a = d.bytes;
+  return s;
+}
+
+// the ids src[0 .. n) of `cols`, in that order, as a compact device dictionary and as a copy in pinned host memory
+// (offsets and bytes, appended to `held`; the copy is complete at the next synchronisation of the stream)
+static int gather_dict(cco_ctx *c, Arena &ar, const StrCols &cols, const uint32_t *src, long long n, DevCol *dev, cco_dictionary_t *host,
+                       std::vector<void *> &held) {
+  cudaStream_t s = c->stream;
+  long long *len, *off;
+  CKR(ar.alloc(&len, n + 1));
+  CKR(ar.alloc(&off, n + 1));
+  CK(cudaMemsetAsync(len + n, 0, 8, s));
+  if (n > 0) {
+    k_ingest_str_lengths<<<grid_for(n, 256, c->sm_count), 256, 0, s>>>(n, cols, src, len);
+    c->launches++;
+  }
+  CKR(exclusive_sum_i64(c, ar, len, off, n + 1));
+  long long total = 0;
+  CKR(mail_fetch(c, &total, off + n, 8));
+  CKR(mail_wait(c));
+  unsigned char *bytes;
+  CKR(ar.alloc(&bytes, std::max<long long>(total, 1)));
+  if (total > 0) {
+    k_ingest_str_gather<<<grid_for(n, 256, c->sm_count), 256, 0, s>>>(n, cols, src, off, bytes);
+    c->launches++;
+  }
+  int64_t *ho = (int64_t *)c->pinned_get(sizeof(int64_t) * ((size_t)n + 1), /*for_result=*/false);
+  if (!ho) return set_error(CCO_E_OOM, "pinned host allocation failed");
+  held.push_back(ho);
+  char *hb = (char *)c->pinned_get((size_t)std::max<long long>(total, 1), /*for_result=*/false);
+  if (!hb) return set_error(CCO_E_OOM, "pinned host allocation failed");
+  held.push_back(hb);
+  CK(cudaMemcpyAsync(ho, off, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyDeviceToHost, s));
+  if (total > 0) CK(cudaMemcpyAsync(hb, bytes, (size_t)total, cudaMemcpyDeviceToHost, s));
+  ar.release(len);
+  dev->n = n;
+  dev->off = off;
+  dev->bytes = bytes;
+  host->n = n;
+  host->offsets = ho;
+  host->bytes = hb;
+  return CCO_OK;
+}
+}  // namespace cco
+
+int cco_ingest_strings(cco_ctx_t *c, int32_t n_types, const cco_string_events_t *ev, int32_t min_events_per_user, uint32_t flags,
+                       cco_dictionary_t *user_dict, cco_dictionary_t *item_dicts, cco_dataset_t **out) {
+  if (!c || !ev || !user_dict || !item_dicts || !out || n_types < 1) return set_error(CCO_E_INVALID_ARG, "null argument or n_types < 1");
+  *out = nullptr;
+  if (!c->members.empty()) return set_error(CCO_E_UNSUPPORTED, "cco_ingest_strings needs a single-GPU context, not a group context");
+  const char *const which[2] = {"user", "item"};
+  for (int t = 0; t < n_types; ++t) {
+    if (ev[t].user.n != ev[t].item.n)
+      return set_error(CCO_E_INVALID_ARG, "type %d: %lld user ids but %lld item ids", t, (long long)ev[t].user.n, (long long)ev[t].item.n);
+    const long long n = ev[t].user.n;
+    if (n < 0 || n >= (1LL << 32)) return set_error(CCO_E_INVALID_ARG, "type %d: %lld events (at most 2^32 - 1 per type)", t, n);
+    for (int w = 0; w < 2; ++w) {
+      const cco_dictionary_t &d = w ? ev[t].item : ev[t].user;
+      if (!d.offsets) return set_error(CCO_E_INVALID_ARG, "type %d: null %s offsets", t, which[w]);
+      if (d.offsets[0] != 0) return set_error(CCO_E_INVALID_ARG, "type %d: %s offsets[0] != 0", t, which[w]);
+      if (d.offsets[n] < 0) return set_error(CCO_E_INVALID_ARG, "type %d: %s offsets decrease", t, which[w]);
+      if (d.offsets[n] > 0 && !d.bytes) return set_error(CCO_E_INVALID_ARG, "type %d: null %s bytes", t, which[w]);
+    }
+  }
+  CK(cudaSetDevice(c->device));
+  cudaStream_t s = c->stream;
+  nvtx_push("cco:ingest_strings");
+  struct Pop { ~Pop() { nvtx_pop(); } } pop;
+  mail_reset(c);
+  Arena ar(s);
+  const bool sh = (flags & CCO_FLAG_INGEST_SHORT_HASH) != 0;
+  // pinned dictionary copies: handed to the caller on success, returned to the pool otherwise
+  struct Held {
+    cco_ctx *c;
+    std::vector<void *> p;
+    bool ok = false;
+    ~Held() {
+      if (!ok)
+        for (void *q : p) c->pinned_put(q);
+    }
+  } held{c};
+  // offsets first: no byte is read before every column's offsets are known not to decrease
+  std::vector<DevCol> col(2 * (size_t)n_types);
+  int *bad;
+  CKR(ar.alloc(&bad, 1));
+  CK(cudaMemsetAsync(bad, 0x7f, sizeof(int), s));
+  for (int t = 0; t < n_types; ++t)
+    for (int w = 0; w < 2; ++w) {
+      const cco_dictionary_t &d = w ? ev[t].item : ev[t].user;
+      DevCol &dc = col[2 * t + w];
+      dc.n = d.n;
+      CKR(ar.alloc(&dc.off, d.n + 1));
+      CK(cudaMemcpyAsync(dc.off, d.offsets, sizeof(int64_t) * ((size_t)d.n + 1), cudaMemcpyHostToDevice, s));
+      if (d.n > 0) {
+        k_ingest_str_check_offsets<<<grid_for(d.n, 256, c->sm_count), 256, 0, s>>>(d.n, dc.off, 2 * t + w, bad);
+        c->launches++;
+      }
+    }
+  int first_bad = 0;
+  CKR(mail_fetch(c, &first_bad, bad, sizeof(int)));
+  CKR(mail_wait(c));
+  if (first_bad != 0x7f7f7f7f) return set_error(CCO_E_INVALID_ARG, "type %d: %s offsets decrease", first_bad / 2, which[first_bad & 1]);
+  for (int t = 0; t < n_types; ++t)
+    for (int w = 0; w < 2; ++w) {
+      const cco_dictionary_t &d = w ? ev[t].item : ev[t].user;
+      DevCol &dc = col[2 * t + w];
+      const long long nb = d.offsets[d.n];
+      CKR(ar.alloc(&dc.bytes, std::max<long long>(nb, 1)));
+      if (nb > 0) CK(cudaMemcpyAsync(dc.bytes, d.bytes, (size_t)nb, cudaMemcpyHostToDevice, s));
+    }
+
+  // users of the primary type: group, count, rank by first appearance
+  std::vector<cco_dictionary_t> host(1 + (size_t)n_types);
+  std::vector<long long *> uraw(n_types, nullptr);
+  std::vector<uint32_t *> surv(n_types, nullptr);
+  std::vector<int32_t *> iraw(n_types, nullptr);
+  std::vector<int32_t> n_items(n_types, 0);
+  const long long n0 = col[0].n;
+  const StrCols u0 = one_column(col[0]);
+  uint32_t *rep0, *cnt, *first, *kept, *fpos, *kpos;
+  CKR(ar.alloc(&rep0, n0));
+  CKR(ar.alloc(&cnt, n0));
+  CKR(ar.alloc(&first, n0 + 1));
+  CKR(ar.alloc(&kept, n0 + 1));
+  CKR(ar.alloc(&fpos, n0 + 1));
+  CKR(ar.alloc(&kpos, n0 + 1));
+  CKR(group_ids(c, ar, n0, u0, sh, rep0));
+  CK(cudaMemsetAsync(cnt, 0, sizeof(uint32_t) * (size_t)std::max<long long>(n0, 1), s));
+  CK(cudaMemsetAsync(first + n0, 0, sizeof(uint32_t), s));
+  CK(cudaMemsetAsync(kept + n0, 0, sizeof(uint32_t), s));
+  const uint32_t need = min_events_per_user > 1 ? (uint32_t)min_events_per_user : 1u;
+  if (n0 > 0) {
+    const int G = grid_for(n0, 256, c->sm_count);
+    k_ingest_str_user_count<<<G, 256, 0, s>>>(n0, rep0, cnt);
+    k_ingest_str_user_flags<<<G, 256, 0, s>>>(n0, rep0, cnt, need, first, kept);
+    c->launches += 2;
+  }
+  CKR(exclusive_sum_u32(c, ar, first, fpos, n0 + 1));
+  CKR(exclusive_sum_u32(c, ar, kept, kpos, n0 + 1));
+  uint32_t n_primary = 0, n_users = 0;
+  CKR(mail_fetch(c, &n_primary, fpos + n0, 4));
+  CKR(mail_fetch(c, &n_users, kpos + n0, 4));
+  CKR(mail_wait(c));
+  if (n_primary > 0x7ffffffeu) return set_error(CCO_E_UNSUPPORTED, "%u distinct primary users (at most 2^31 - 2)", n_primary);
+  uint32_t *dict_ev, *dict_raw;
+  CKR(ar.alloc(&dict_ev, n_users));
+  CKR(ar.alloc(&dict_raw, n_users));
+  CKR(ar.alloc(&uraw[0], n0));
+  CKR(ar.alloc(&surv[0], n0));
+  if (n0 > 0) {
+    k_ingest_str_user_tokens<<<grid_for(n0, 256, c->sm_count), 256, 0, s>>>(n0, rep0, fpos, kept, kpos, uraw[0], surv[0], dict_ev, dict_raw);
+    c->launches++;
+  }
+  DevCol udict;
+  CKR(gather_dict(c, ar, u0, dict_ev, n_users, &udict, &host[0], held.p));
+  for (void *p : {(void *)rep0, (void *)cnt, (void *)first, (void *)kept, (void *)fpos, (void *)kpos, (void *)dict_ev}) ar.release(p);
+
+  // users of the other types: grouped together with the user dictionary (elements [0, n_users)), in chunks that keep
+  // the element count below 2^32
+  for (int t = 1; t < n_types; ++t) {
+    const long long n = col[2 * t].n;
+    CKR(ar.alloc(&uraw[t], n));
+    CKR(ar.alloc(&surv[t], n));
+    const long long kChunk = 1LL << 31;
+    for (long long c0 = 0; c0 < n; c0 += kChunk) {
+      const long long m = std::min(kChunk, n - c0);
+      StrCols sc = one_column(udict);
+      sc.off_b = col[2 * t].off + c0;
+      sc.bytes_b = col[2 * t].bytes;
+      uint32_t *rep;
+      CKR(ar.alloc(&rep, n_users + m));
+      CKR(group_ids(c, ar, n_users + m, sc, sh, rep));
+      k_ingest_str_match_users<<<grid_for(m, 256, c->sm_count), 256, 0, s>>>(m, n_users, rep, dict_raw, n_primary, uraw[t] + c0,
+                                                                            surv[t] + c0);
+      c->launches++;
+      ar.release(rep);
+    }
+  }
+
+  // items of every type: group, rank by first surviving appearance
+  for (int t = 0; t < n_types; ++t) {
+    const DevCol &ic = col[2 * t + 1];
+    const long long n = ic.n;
+    const StrCols cols = one_column(ic);
+    uint32_t *rep, *fs, *flag, *ipos;
+    CKR(ar.alloc(&iraw[t], n));
+    CKR(ar.alloc(&rep, n));
+    CKR(ar.alloc(&fs, n));
+    CKR(ar.alloc(&flag, n + 1));
+    CKR(ar.alloc(&ipos, n + 1));
+    CKR(group_ids(c, ar, n, cols, sh, rep));
+    CK(cudaMemsetAsync(fs, 0xff, sizeof(uint32_t) * (size_t)std::max<long long>(n, 1), s));
+    CK(cudaMemsetAsync(flag + n, 0, sizeof(uint32_t), s));
+    if (n > 0) {
+      const int G = grid_for(n, 256, c->sm_count);
+      k_ingest_str_first_surv<<<G, 256, 0, s>>>(n, rep, surv[t], fs);
+      k_ingest_str_item_flags<<<G, 256, 0, s>>>(n, rep, fs, flag);
+      c->launches += 2;
+    }
+    CKR(exclusive_sum_u32(c, ar, flag, ipos, n + 1));
+    uint32_t q = 0;
+    CKR(mail_fetch(c, &q, ipos + n, 4));
+    CKR(mail_wait(c));
+    if (q > 0x7ffffffeu) return set_error(CCO_E_UNSUPPORTED, "type %d: %u distinct items (at most 2^31 - 2)", t, q);
+    n_items[t] = (int32_t)q;
+    uint32_t *idict;
+    CKR(ar.alloc(&idict, q));
+    if (n > 0) {
+      k_ingest_str_item_tokens<<<grid_for(n, 256, c->sm_count), 256, 0, s>>>(n, rep, surv[t], fs, flag, ipos, iraw[t], idict);
+      c->launches++;
+    }
+    DevCol idev;
+    CKR(gather_dict(c, ar, cols, idict, q, &idev, &host[1 + t], held.p));
+    for (void *p : {(void *)rep, (void *)fs, (void *)flag, (void *)ipos, (void *)idict, (void *)ic.off, (void *)ic.bytes}) ar.release(p);
+  }
+
+  // the matrices: raw user id n_primary has no primary event, so the users unknown to the dictionary drop out there
+  IngestSource src;
+  src.n_types = n_types;
+  src.n_users_raw = (long long)n_primary + 1;
+  for (int t = 0; t < n_types; ++t) {
+    src.n_events.push_back(col[2 * t].n);
+    src.n_items_raw.push_back(n_items[t]);
+  }
+  src.fill = [&](int t, long long *d_user, int32_t *d_item) -> int {
+    const size_t n = (size_t)col[2 * t].n;
+    CK(cudaMemcpyAsync(d_user, uraw[t], sizeof(int64_t) * n, cudaMemcpyDeviceToDevice, s));
+    CK(cudaMemcpyAsync(d_item, iraw[t], sizeof(int32_t) * n, cudaMemcpyDeviceToDevice, s));
+    return CCO_OK;
+  };
+  cco_dataset *d = nullptr;
+  CKR(ingest_core(c, src, min_events_per_user, nullptr, nullptr, &d));   // ends in a stream synchronise: the dictionaries are home
+  held.ok = true;
+  *user_dict = host[0];
+  for (int t = 0; t < n_types; ++t) item_dicts[t] = host[1 + t];
+  *out = d;
+  return CCO_OK;
 }
 
 // copy matrix i of a resident dataset into caller-provided host arrays (pinned ones from cco_host_alloc copy at PCIe speed)

@@ -2,8 +2,8 @@
 (/root/reference/src/main/scala/Preparator.scala:44-87, 100-216): event (user, item) string pairs
 per event name -> IndexedDatasets that share one user dictionary.
 
-This is the INPUT side of the hot-path boundary (SURVEY.md 8a-H1); it is host logic in numpy and
-is listed as the next row to move to the device (SURVEY.md 8f-1)."""
+This is the INPUT side of the hot-path boundary (SURVEY.md 8a-H1).  `prepare` is the host logic;
+`prepare_on_device` gives the same result from the same id strings through cco_ingest_strings (SURVEY.md 8f-1)."""
 from __future__ import annotations
 
 from typing import Sequence
@@ -66,3 +66,34 @@ def prepare(actions: Sequence[tuple[str, Sequence[tuple[str, str]]]],
         user_dict = ids.row_ids
         out.append((name, ids))
     return out
+
+
+def encode_ids(ids: Sequence[str]) -> tuple[np.ndarray, np.ndarray]:
+    """id strings -> (offsets int64[n + 1], UTF-8 bytes uint8[]): id e = bytes[offsets[e]:offsets[e + 1]].  Vectorised:
+    one join, one UTF-8 and one UTF-32 encode of the whole column; the UTF-8 length of every code point gives the offsets."""
+    n = len(ids)
+    joined = "".join(ids)
+    data = np.frombuffer(joined.encode("utf-8"), dtype=np.uint8)
+    cps = np.frombuffer(joined.encode("utf-32-le"), dtype=np.uint32)
+    cp_bytes = np.zeros(len(cps) + 1, dtype=np.int64)
+    np.cumsum(1 + (cps >= 0x80) + (cps >= 0x800) + (cps >= 0x10000), out=cp_bytes[1:])
+    chars = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(np.fromiter(map(len, ids), dtype=np.int64, count=n), out=chars[1:])
+    return cp_bytes[chars], data
+
+
+def prepare_on_device(ctx, actions: Sequence[tuple[str, Sequence[tuple[str, str]]]],
+                      min_events_per_user: int | None = None):
+    """`prepare` on the B200 (cco_ingest_strings): same arguments and the same [(name, IndexedDataset)], plus the
+    HBM-resident dataset the matrices came from, ready for ctx.train_dataset (release it with ctx.free_dataset)."""
+    types = []
+    for _, pairs in actions:
+        users, items = zip(*pairs) if len(pairs) else ((), ())
+        types.append((*encode_ids(users), *encode_ids(items)))
+    ds, user_ids, item_ids = ctx.ingest_strings(types, min_events_per_user or 0)
+    row_ids = BiDictionary(user_ids)
+    out = []
+    for t, (name, _) in enumerate(actions):
+        nr, nc, rp, ci = ctx.dataset_matrix(ds, t)
+        out.append((name, IndexedDataset(rp, ci, row_ids, BiDictionary(item_ids[t]), n_rows=nr, n_cols=nc)))
+    return out, ds

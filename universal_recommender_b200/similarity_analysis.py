@@ -238,11 +238,12 @@ class CcoContext:
         N.check(self._L.cco_dataset_upload(self._h, len(mats), cm, flags, C.byref(ds)))
         return (ds, len(mats))
 
-    def train_dataset(self, dataset, params, seed: int, flags: int = 0, copy_arrays: bool = True):
+    def train_dataset(self, dataset, params, seed: int, flags: int = 0, copy_arrays: bool = True, keep: bool = False):
+        """keep=True: as for train_csr, zero-copy views + a handle for free_result / format_es_bulk."""
         ds, n = dataset
         res = C.c_void_p()
         N.check(self._L.cco_train_dataset(self._h, ds, self._params_array(params), C.c_int32(_to_i32(seed)), flags, C.byref(res)))
-        return self._collect(res, n, copy_arrays)
+        return self._collect(res, n, copy_arrays, keep)
 
     def ingest(self, events, n_users_raw: int, min_events_per_user: int = 0):
         """Preparator.prepare on the device (SURVEY.md 8f-1).  events = [(users int64[], items int32[], n_items_raw)], type 0
@@ -261,6 +262,37 @@ class CcoContext:
         N.check(self._L.cco_ingest(self._h, n, ev, n_users_raw, min_events_per_user, user_map.ctypes.data_as(C.POINTER(C.c_int32)),
                                    maps, C.byref(ds)))
         return (ds, n), user_map[:n_users_raw], [m[:ni] for m, (_, _, ni) in zip(item_maps, events)]
+
+    def ingest_strings(self, types, min_events_per_user: int = 0, flags: int = 0):
+        """Preparator.prepare on the device from raw id strings (cco_ingest_strings).  types = [(user_offsets int64[],
+        user_bytes uint8[], item_offsets int64[], item_bytes uint8[])], type 0 = primary; the ids of event e are
+        bytes[offsets[e]:offsets[e + 1]].  -> (dataset for train_dataset, user ids, [item ids of each type]), the ids as
+        `str` (UTF-8; bytes that are not UTF-8 come back as surrogate escapes) in dictionary order."""
+        n = len(types)
+        keep, ev = [], (N.StringEventsT * n)()
+
+        def column(off, data):
+            off = np.ascontiguousarray(off, dtype=np.int64)
+            data = np.ascontiguousarray(data, dtype=np.uint8)
+            keep.append((off, data))
+            return N.DictionaryRawT(len(off) - 1, off.ctypes.data_as(C.POINTER(C.c_int64)), data.ctypes.data if len(data) else None)
+
+        for t, (uo, ub, io, ib) in enumerate(types):
+            ev[t] = N.StringEventsT(column(uo, ub), column(io, ib))
+        user, items = N.DictionaryRawT(), (N.DictionaryRawT * n)()
+        ds = C.c_void_p()
+        N.check(self._L.cco_ingest_strings(self._h, n, ev, int(min_events_per_user), flags, C.byref(user), items, C.byref(ds)))
+        return (ds, n), self._take_ids(user), [self._take_ids(items[t]) for t in range(n)]
+
+    def _take_ids(self, d) -> list[str]:
+        """decode a dictionary the library returned in pinned memory, then hand the memory back"""
+        try:
+            off = np.ctypeslib.as_array(d.offsets, shape=(d.n + 1,)).tolist()
+            blob = C.string_at(d.bytes, off[-1]) if off[-1] else b""
+            return [blob[a:b].decode("utf-8", "surrogateescape") for a, b in zip(off, off[1:])]
+        finally:
+            self._L.cco_host_free(self._h, C.cast(d.offsets, C.c_void_p))
+            self._L.cco_host_free(self._h, d.bytes)
 
     def synth_dataset(self, types, n_users_raw: int, user_cdf: np.ndarray, user_perm: np.ndarray, min_events_per_user: int = 0,
                       raw_item_space: bool = False):
