@@ -333,6 +333,47 @@ int cco_pop_model(cco_ctx_t *ctx, int32_t mode, int64_t n_events, const int32_t 
                   int64_t start_ms, int64_t end_ms, double *score, unsigned char *present);
 
 /*
+ * The whole model document as URModel.save writes it with recsModel "all" (src/main/scala/URAlgorithm.scala:351-367,
+ * 537-560; URModel.scala:57-102): groupAll(correlators ++ propertiesRDD), where propertiesRDD is the item properties
+ * full-outer-joined with one rank field per ranking.  Rankings and property ids join the model rows by their id strings.
+ *  - Documents: one per model row, in row order, then one per extra id in order of first appearance in the sequence
+ *    (ranking 0's events, ranking 1's, ..., property ids).  An extra id is not a row and has a present rank in at least one
+ *    ranking or a property entry.  An id seen only in rankings where it is not present (trending / hot inner joins, the
+ *    empty-bucket rules) gets no document.
+ *  - Fields, in this order: "id"; for rows only, the indicator arrays exactly as cco_format_es_bulk writes them;
+ *    ,"<ranking name>":<score> for each ranking in which the id is present; ,<fragment> if the id's property fragment is
+ *    not empty.  The action line is {"index":{"_id":"<id>"}} as in cco_format_es_bulk.
+ *  - A property fragment is JSON object members without braces ("categories":["Phones"],"available":"2017-..."),
+ *    serialised by the caller and spliced in verbatim: $set properties, userDefined ranks, random ranks.
+ *  - Scores are the histograms of cco_pop_model (same bucket edges, same empty-bucket rules): integral doubles written as
+ *    Java's Double.toString writes them: "<int>.0" when |v| < 10^7, otherwise d.dddE<n> with the trailing zeros of the
+ *    fraction stripped and at least one fractional digit (1.0E7, 1.2345678E7, -8.589934592E9).
+ *  - Ids are equal iff their bytes are equal.  With n_rankings == 0 and no properties the output is byte-identical to
+ *    cco_format_es_bulk.
+ * ranking.item holds the item id of every event of the ranking's event names (any user, any time); time_ms[e] is event
+ * e's time in epoch milliseconds.  prop_ids and prop_json are both NULL or both given with the same n.  flags accepts
+ * CCO_FLAG_INGEST_SHORT_HASH (tests only).  A group context formats on its first GPU.  *out_bytes is pinned memory owned by
+ * the context: release it with cco_host_free.
+ * Errors: CCO_E_INVALID_ARG for null pointers, only one of prop_ids / prop_json, row_ids.n != the model's row count, bad
+ * offsets in any dictionary (checked before any id byte is read), end_ms < start_ms, a bad mode, a ranking name that is
+ * null, repeated, "id" or an indicator name, two equal ids in row_ids, two equal ids in prop_ids.  CCO_E_UNSUPPORTED for a
+ * result that is one rank's row slice (extra documents would repeat across ranks), more than 3 rankings, 2^31 or more
+ * events in a ranking, 2^32 or more ids in all, or 2^31 or more distinct ids.
+ */
+typedef struct {
+  const char *name;         /* ES field, e.g. "popRank" */
+  int32_t mode;             /* CCO_POP_POPULAR / _TRENDING / _HOT */
+  int32_t reserved;
+  int64_t start_ms, end_ms; /* [end - duration, end), as cco_pop_model */
+  cco_dictionary_t item;    /* the item id of every event of the ranking's event names */
+  const int64_t *time_ms;   /* [item.n] event times */
+} cco_ranking_t;
+int cco_format_model_bulk(cco_ctx_t *ctx, const cco_result_t *res, int32_t n_names, const char *const *names,
+                          const cco_dictionary_t *row_ids, const cco_dictionary_t *col_ids, int32_t n_rankings,
+                          const cco_ranking_t *rankings, const cco_dictionary_t *prop_ids, const cco_dictionary_t *prop_json,
+                          uint32_t flags, char **out_bytes, int64_t *out_len);
+
+/*
  * Debug/parity entry (tests only): full integer co-occurrence matrix A^T B of two canonical
  * binary matrices computed by the same accumulation kernel as cco_train, no LLR, no top-k.
  * Output CSR over the columns of A with ascending column ids, malloc'ed; free with cco_free.

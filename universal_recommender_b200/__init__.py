@@ -9,6 +9,7 @@ Host-side mirror of the reference interface for this path:
   DownsamplableCrossOccurrenceDataset     <- URAlgorithm.scala:336-340
   SimilarityAnalysis.cooccurrencesIDSs / crossOccurrenceDownsampled  <- URAlgorithm.scala:323,343
   ur_algorithm.calc_all                   <- URAlgorithm.calcAll          (URAlgorithm.scala:310-349)
+  ur_algorithm.write_model                <- the documents calcAll hands to URModel.save (URAlgorithm.scala:351-367)
 """
 from ._native import (CcoError, CcoInvalidArgument, FLAG_ASSUME_CANONICAL, FLAG_ENTROPY_VARARGS, FLAG_RESULT_NO_COUNT,
                       FLAG_RESULT_NO_LLR, FLAG_ROWRATE_INTDIV, LIB_PATH)
@@ -16,11 +17,12 @@ from .indexed_dataset import BiDictionary, IndexedDataset
 from .preparator import prepare, prepare_on_device
 from .similarity_analysis import (CcoContext, DownsamplableCrossOccurrenceDataset, SimilarityAnalysis,
                                   default_context)
-from .ur_algorithm import DefaultURAlgoParams, IndicatorParams, URAlgorithmParams, calc_all
+from .ur_algorithm import (DefaultURAlgoParams, IndicatorParams, RankingParams, URAlgorithmParams, calc_all, resolve_rankings,
+                           write_model)
 
 __all__ = [
     "BiDictionary", "CcoContext", "CcoError", "CcoInvalidArgument", "DefaultURAlgoParams",
-    "DownsamplableCrossOccurrenceDataset", "IndexedDataset", "IndicatorParams", "SimilarityAnalysis",
-    "URAlgorithmParams", "calc_all", "default_context", "prepare", "prepare_on_device", "FLAG_ASSUME_CANONICAL",
+    "DownsamplableCrossOccurrenceDataset", "IndexedDataset", "IndicatorParams", "RankingParams", "SimilarityAnalysis",
+    "URAlgorithmParams", "calc_all", "resolve_rankings", "write_model", "default_context", "prepare", "prepare_on_device", "FLAG_ASSUME_CANONICAL",
     "FLAG_ENTROPY_VARARGS", "FLAG_ROWRATE_INTDIV", "FLAG_RESULT_NO_COUNT", "FLAG_RESULT_NO_LLR", "LIB_PATH",
 ]

@@ -71,6 +71,11 @@ class StringEventsT(C.Structure):
     _fields_ = [("user", DictionaryRawT), ("item", DictionaryRawT)]
 
 
+class RankingT(C.Structure):
+    _fields_ = [("name", C.c_char_p), ("mode", C.c_int32), ("reserved", C.c_int32), ("start_ms", C.c_int64), ("end_ms", C.c_int64),
+                ("item", DictionaryRawT), ("time_ms", C.POINTER(C.c_int64))]
+
+
 class StatsT(C.Structure):
     _fields_ = [("n_users", C.c_int64), ("nnz_in_total", C.c_int64),
                 ("nnz_downsampled", C.c_int64 * 16), ("products", C.c_int64 * 16),
@@ -86,7 +91,7 @@ EXPORTS = [
     "cco_create", "cco_create_group", "cco_destroy", "cco_host_alloc", "cco_host_free", "cco_train", "cco_cooccurrences_idss",
     "cco_dataset_upload", "cco_train_dataset", "cco_dataset_free", "cco_timer_start", "cco_timer_stop",
     "cco_partition_rows", "cco_ingest", "cco_synth_ingest", "cco_dataset_shape", "cco_dataset_download",
-    "cco_dataset_copy_to_host", "cco_format_es_bulk", "cco_ingest_strings", "cco_pop_model",
+    "cco_dataset_copy_to_host", "cco_format_es_bulk", "cco_format_model_bulk", "cco_ingest_strings", "cco_pop_model",
     "cco_result_num_matrices", "cco_result_row_range", "cco_result_matrix", "cco_result_stats", "cco_result_free",
     "cco_debug_cooccurrence", "cco_debug_downsample", "cco_debug_llr", "cco_free",
 ]
@@ -127,6 +132,8 @@ def lib():
     L.cco_dataset_copy_to_host.argtypes = [C.c_void_p, C.c_int32, p(C.c_int64), p(C.c_int32)]
     L.cco_format_es_bulk.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, p(C.c_char_p), p(DictionaryT), p(DictionaryT), p(C.c_void_p),
                                      p(C.c_int64)]
+    L.cco_format_model_bulk.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, p(C.c_char_p), p(DictionaryRawT), p(DictionaryRawT), C.c_int32,
+                                        p(RankingT), p(DictionaryRawT), p(DictionaryRawT), C.c_uint32, p(C.c_void_p), p(C.c_int64)]
     L.cco_ingest_strings.argtypes = [C.c_void_p, C.c_int32, p(StringEventsT), C.c_int32, C.c_uint32, p(DictionaryRawT),
                                      p(DictionaryRawT), p(C.c_void_p)]
     L.cco_pop_model.argtypes = [C.c_void_p, C.c_int32, C.c_int64, p(C.c_int32), p(C.c_int64), C.c_int32, C.c_int64, C.c_int64, p(C.c_double),

@@ -25,6 +25,7 @@
 #include "cco_sampler.cuh"
 #include "cco_format.cuh"
 #include "cco_strings.cuh"
+#include "cco_model.cuh"
 
 namespace cco {
 
@@ -2098,8 +2099,8 @@ static StrCols one_column(const DevCol &d) {
   return s;
 }
 
-// the ids src[0 .. n) of `cols`, in that order, as a compact device dictionary and as a copy in pinned host memory
-// (offsets and bytes, appended to `held`; the copy is complete at the next synchronisation of the stream)
+// the ids src[0 .. n) of `cols`, in that order, as a compact device dictionary and, unless host is null, as a copy in pinned
+// host memory (offsets and bytes, appended to `held`; the copy is complete at the next synchronisation of the stream)
 static int gather_dict(cco_ctx *c, Arena &ar, const StrCols &cols, const uint32_t *src, long long n, DevCol *dev, cco_dictionary_t *host,
                        std::vector<void *> &held) {
   cudaStream_t s = c->stream;
@@ -2121,6 +2122,11 @@ static int gather_dict(cco_ctx *c, Arena &ar, const StrCols &cols, const uint32_
     k_ingest_str_gather<<<grid_for(n, 256, c->sm_count), 256, 0, s>>>(n, cols, src, off, bytes);
     c->launches++;
   }
+  ar.release(len);
+  dev->n = n;
+  dev->off = off;
+  dev->bytes = bytes;
+  if (!host) return CCO_OK;
   int64_t *ho = (int64_t *)c->pinned_get(sizeof(int64_t) * ((size_t)n + 1), /*for_result=*/false);
   if (!ho) return set_error(CCO_E_OOM, "pinned host allocation failed");
   held.push_back(ho);
@@ -2129,10 +2135,6 @@ static int gather_dict(cco_ctx *c, Arena &ar, const StrCols &cols, const uint32_
   held.push_back(hb);
   CK(cudaMemcpyAsync(ho, off, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyDeviceToHost, s));
   if (total > 0) CK(cudaMemcpyAsync(hb, bytes, (size_t)total, cudaMemcpyDeviceToHost, s));
-  ar.release(len);
-  dev->n = n;
-  dev->off = off;
-  dev->bytes = bytes;
   host->n = n;
   host->offsets = ho;
   host->bytes = hb;
@@ -2492,15 +2494,12 @@ static int escape_dict(cco_ctx *c, Arena &ar, const DevDict &raw, DevDict *esc) 
   ar.release(len);
   return CCO_OK;
 }
-}  // namespace cco
 
-int cco_format_es_bulk(cco_ctx_t *ctx, const cco_result_t *res, int32_t n_names, const char *const *names,
-                       const cco_dictionary_t *row_ids, const cco_dictionary_t *col_ids, char **out_bytes, int64_t *out_len) {
-  if (!ctx || !res || !names || !row_ids || !col_ids || !out_bytes || !out_len) return set_error(CCO_E_INVALID_ARG, "null argument");
+// the argument checks cco_format_es_bulk and cco_format_model_bulk share
+static int check_indicators(const cco_result_t *res, int32_t n_names, const char *const *names, const cco_dictionary_t *col_ids) {
   const int n_ind = (int)res->mats.size();
   if (n_names != n_ind) return set_error(CCO_E_INVALID_ARG, "%d event names for %d indicators", n_names, n_ind);
   if (n_ind < 1 || n_ind > kMaxFormatIndicators) return set_error(CCO_E_UNSUPPORTED, "1..%d indicators", kMaxFormatIndicators);
-  cco_ctx *c = ctx->members.empty() ? ctx : ctx->members[0];   // a group's merged model is formatted on its first GPU
   const int64_t row_lo = res->mats[0].row_begin, row_hi = res->mats[0].row_end;
   for (int i = 0; i < n_ind; ++i) {
     const ResultMat &m = res->mats[i];
@@ -2509,43 +2508,45 @@ int cco_format_es_bulk(cco_ctx_t *ctx, const cco_result_t *res, int32_t n_names,
     if (col_ids[i].n < m.n_cols) return set_error(CCO_E_INVALID_ARG, "column dictionary %d has %lld ids for %d columns", i, (long long)col_ids[i].n, m.n_cols);
     if (!names[i]) return set_error(CCO_E_INVALID_ARG, "null event name");
   }
-  if (row_ids->n < row_hi) return set_error(CCO_E_INVALID_ARG, "row dictionary has %lld ids, rows go up to %lld", (long long)row_ids->n, (long long)row_hi);
-  CK(cudaSetDevice(c->device));
-  cudaStream_t s = c->stream;
-  Arena ar(s);
-  nvtx_push("cco:format_es_bulk");
-  struct Pop { ~Pop() { nvtx_pop(); } } pop;
-  FormatArgs fa;
-  memset(&fa, 0, sizeof fa);
-  fa.n_rows = (int32_t)(row_hi - row_lo);
-  fa.row_id_base = row_lo;
-  fa.n_ind = n_ind;
-  DevDict raw;
-  CKR(upload_dict(c, ar, *row_ids, &raw));
-  CKR(escape_dict(c, ar, raw, &fa.row_ids));
-  // event names as one more tiny dictionary
-  {
-    std::vector<int64_t> noff(n_ind + 1, 0);
-    std::string blob;
-    for (int i = 0; i < n_ind; ++i) {
-      blob += names[i];
-      noff[i + 1] = (int64_t)blob.size();
-    }
-    cco_dictionary_t nd = {n_ind, noff.data(), blob.data()};
-    DevDict nraw, nesc;
-    CKR(upload_dict(c, ar, nd, &nraw));
-    CK(cudaStreamSynchronize(s));   // noff / blob are locals
-    CKR(escape_dict(c, ar, nraw, &nesc));
-    std::vector<long long> eoff(n_ind + 1);
-    CK(cudaMemcpyAsync(eoff.data(), nesc.off, sizeof(long long) * ((size_t)n_ind + 1), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    fa.names = nesc.bytes;
-    for (int i = 0; i <= n_ind; ++i) fa.name_off[i] = (int32_t)eoff[i];
+  return CCO_OK;
+}
+
+// n C strings as one escaped blob on the device: string i = bytes[off[i] .. off[i + 1])
+static int escape_names(cco_ctx *c, Arena &ar, int n, const char *const *names, const unsigned char **bytes, int32_t *off) {
+  std::vector<int64_t> noff(n + 1, 0);
+  std::string blob;
+  for (int i = 0; i < n; ++i) {
+    blob += names[i];
+    noff[i + 1] = (int64_t)blob.size();
   }
+  cco_dictionary_t nd = {n, noff.data(), blob.data()};
+  DevDict nraw, nesc;
+  CKR(upload_dict(c, ar, nd, &nraw));
+  CK(cudaStreamSynchronize(c->stream));   // noff / blob are locals
+  CKR(escape_dict(c, ar, nraw, &nesc));
+  std::vector<long long> eoff(n + 1);
+  CK(cudaMemcpyAsync(eoff.data(), nesc.off, sizeof(long long) * ((size_t)n + 1), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  *bytes = nesc.bytes;
+  for (int i = 0; i <= n; ++i) off[i] = (int32_t)eoff[i];
+  return CCO_OK;
+}
+
+// the indicator part of FormatArgs on the device: event names and column dictionaries escaped, the rows of every indicator
+static int upload_indicators(cco_ctx *c, Arena &ar, const cco_result_t *res, const char *const *names, const cco_dictionary_t *col_ids,
+                             FormatArgs *fa) {
+  cudaStream_t s = c->stream;
+  const int n_ind = (int)res->mats.size();
+  const int64_t row_lo = res->mats[0].row_begin, row_hi = res->mats[0].row_end;
+  fa->n_rows = (int32_t)(row_hi - row_lo);
+  fa->row_id_base = row_lo;
+  fa->n_ind = n_ind;
+  CKR(escape_names(c, ar, n_ind, names, &fa->names, fa->name_off));
   for (int i = 0; i < n_ind; ++i) {
     const ResultMat &m = res->mats[i];
+    DevDict raw;
     CKR(upload_dict(c, ar, col_ids[i], &raw));
-    CKR(escape_dict(c, ar, raw, &fa.col_ids[i]));
+    CKR(escape_dict(c, ar, raw, &fa->col_ids[i]));
     const long long n_my = row_hi - row_lo, nnz = m.row_ptr[n_my] - m.row_ptr[0];
     long long *d_rp;
     int32_t *d_col;
@@ -2557,28 +2558,38 @@ int cco_format_es_bulk(cco_ctx_t *ctx, const cco_result_t *res, int32_t n_names,
       k_add_i64<<<grid_for(n_my + 1, 256, c->sm_count, 2), 256, 0, s>>>(n_my + 1, -(long long)m.row_ptr[0], d_rp);
       c->launches++;
     }
-    fa.row_ptr[i] = d_rp;
-    fa.col[i] = d_col;
+    fa->row_ptr[i] = d_rp;
+    fa->col[i] = d_col;
   }
+  return CCO_OK;
+}
+
+// lengths of n_docs documents -> exclusive scan -> bytes, copied into pinned memory of `owner` (the caller frees it with
+// cco_host_free).  launch_len(doc_len) and launch_write(doc_off, out) enqueue the two kernels.
+extern "C++" {   // a template inside the extern "C" block of the entries
+template <class Len, class Write>
+static int assemble_docs(cco_ctx *owner, cco_ctx *c, Arena &ar, long long n_docs, Len launch_len, Write launch_write, char **out_bytes,
+                         int64_t *out_len) {
+  cudaStream_t s = c->stream;
   long long *doc_len, *doc_off;
-  CKR(ar.alloc(&doc_len, fa.n_rows + 1));
-  CKR(ar.alloc(&doc_off, fa.n_rows + 1));
-  CK(cudaMemsetAsync(doc_len + fa.n_rows, 0, 8, s));
-  if (fa.n_rows > 0) {
-    k_doc_len<<<grid_for(fa.n_rows, 256, c->sm_count), 256, 0, s>>>(fa, doc_len);
+  CKR(ar.alloc(&doc_len, n_docs + 1));
+  CKR(ar.alloc(&doc_off, n_docs + 1));
+  CK(cudaMemsetAsync(doc_len + n_docs, 0, 8, s));
+  if (n_docs > 0) {
+    launch_len(doc_len);
     c->launches++;
   }
-  CKR(exclusive_sum_i64(c, ar, doc_len, doc_off, (long long)fa.n_rows + 1));
+  CKR(exclusive_sum_i64(c, ar, doc_len, doc_off, n_docs + 1));
   long long total = 0;
-  CK(cudaMemcpyAsync(&total, doc_off + fa.n_rows, 8, cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(&total, doc_off + n_docs, 8, cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
   unsigned char *d_out;
   CKR(ar.alloc(&d_out, std::max<long long>(total, 1)));
-  if (fa.n_rows > 0 && total > 0) {
-    k_doc_write<<<grid_for((long long)fa.n_rows * 32, 256, c->sm_count), 256, 0, s>>>(fa, doc_off, d_out);
+  if (n_docs > 0 && total > 0) {
+    launch_write(doc_off, d_out);
     c->launches++;
   }
-  char *host = (char *)ctx->pinned_get((size_t)std::max<long long>(total, 1), /*for_result=*/false);
+  char *host = (char *)owner->pinned_get((size_t)std::max<long long>(total, 1), /*for_result=*/false);
   if (!host) return set_error(CCO_E_OOM, "pinned host allocation failed");
   if (total > 0) CK(cudaMemcpyAsync(host, d_out, (size_t)total, cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
@@ -2587,21 +2598,10 @@ int cco_format_es_bulk(cco_ctx_t *ctx, const cco_result_t *res, int32_t n_names,
   *out_len = total;
   return CCO_OK;
 }
+}  // extern "C++"
 
-// ---- SURVEY.md 8f-3: PopModel rank histograms -------------------------------------------------------------------------
-int cco_pop_model(cco_ctx_t *ctx, int32_t mode, int64_t n_events, const int32_t *item, const int64_t *time_ms, int32_t n_items,
-                  int64_t start_ms, int64_t end_ms, double *score, unsigned char *present) {
-  if (!ctx || n_events < 0 || n_items < 0 || (n_events > 0 && (!item || !time_ms)) || (n_items > 0 && (!score || !present)))
-    return set_error(CCO_E_INVALID_ARG, "bad argument");
-  if (mode < CCO_POP_POPULAR || mode > CCO_POP_HOT) return set_error(CCO_E_INVALID_ARG, "mode must be CCO_POP_POPULAR, _TRENDING or _HOT");
-  if (end_ms < start_ms) return set_error(CCO_E_INVALID_ARG, "end before start (Joda Interval would throw)");
-  if (n_items == 0) return CCO_OK;
-  cco_ctx *c = ctx->members.empty() ? ctx : ctx->members[0];
-  CK(cudaSetDevice(c->device));
-  cudaStream_t s = c->stream;
-  Arena ar(s);
-  nvtx_push("cco:pop_model");
-  struct Pop { ~Pop() { nvtx_pop(); } } pop;
+// PopModel's bucket edges: Joda's integer millisecond arithmetic over [start_ms, end_ms)
+static PopArgs pop_args(int32_t mode, int64_t start_ms, int64_t end_ms, int32_t n_items) {
   PopArgs a;
   memset(&a, 0, sizeof a);
   a.n_items = n_items;
@@ -2622,6 +2622,52 @@ int cco_pop_model(cco_ctx_t *ctx, int32_t mode, int64_t n_events, const int32_t 
     a.edge[2] = a.edge[1] + dur / 3;
     a.edge[3] = end_ms;
   }
+  return a;
+}
+}  // namespace cco
+
+int cco_format_es_bulk(cco_ctx_t *ctx, const cco_result_t *res, int32_t n_names, const char *const *names,
+                       const cco_dictionary_t *row_ids, const cco_dictionary_t *col_ids, char **out_bytes, int64_t *out_len) {
+  if (!ctx || !res || !names || !row_ids || !col_ids || !out_bytes || !out_len) return set_error(CCO_E_INVALID_ARG, "null argument");
+  CKR(check_indicators(res, n_names, names, col_ids));
+  cco_ctx *c = ctx->members.empty() ? ctx : ctx->members[0];   // a group's merged model is formatted on its first GPU
+  const int64_t row_hi = res->mats[0].row_end;
+  if (row_ids->n < row_hi) return set_error(CCO_E_INVALID_ARG, "row dictionary has %lld ids, rows go up to %lld", (long long)row_ids->n, (long long)row_hi);
+  CK(cudaSetDevice(c->device));
+  cudaStream_t s = c->stream;
+  Arena ar(s);
+  nvtx_push("cco:format_es_bulk");
+  struct Pop { ~Pop() { nvtx_pop(); } } pop;
+  FormatArgs fa;
+  memset(&fa, 0, sizeof fa);
+  DevDict raw;
+  CKR(upload_dict(c, ar, *row_ids, &raw));
+  CKR(escape_dict(c, ar, raw, &fa.row_ids));
+  CKR(upload_indicators(c, ar, res, names, col_ids, &fa));
+  return assemble_docs(
+      ctx, c, ar, fa.n_rows,
+      [&](long long *doc_len) { k_doc_len<<<grid_for(fa.n_rows, 256, c->sm_count), 256, 0, s>>>(fa, doc_len); },
+      [&](const long long *doc_off, unsigned char *out) {
+        k_doc_write<<<grid_for((long long)fa.n_rows * 32, 256, c->sm_count), 256, 0, s>>>(fa, doc_off, out);
+      },
+      out_bytes, out_len);
+}
+
+// ---- SURVEY.md 8f-3: PopModel rank histograms -------------------------------------------------------------------------
+int cco_pop_model(cco_ctx_t *ctx, int32_t mode, int64_t n_events, const int32_t *item, const int64_t *time_ms, int32_t n_items,
+                  int64_t start_ms, int64_t end_ms, double *score, unsigned char *present) {
+  if (!ctx || n_events < 0 || n_items < 0 || (n_events > 0 && (!item || !time_ms)) || (n_items > 0 && (!score || !present)))
+    return set_error(CCO_E_INVALID_ARG, "bad argument");
+  if (mode < CCO_POP_POPULAR || mode > CCO_POP_HOT) return set_error(CCO_E_INVALID_ARG, "mode must be CCO_POP_POPULAR, _TRENDING or _HOT");
+  if (end_ms < start_ms) return set_error(CCO_E_INVALID_ARG, "end before start (Joda Interval would throw)");
+  if (n_items == 0) return CCO_OK;
+  cco_ctx *c = ctx->members.empty() ? ctx : ctx->members[0];
+  CK(cudaSetDevice(c->device));
+  cudaStream_t s = c->stream;
+  Arena ar(s);
+  nvtx_push("cco:pop_model");
+  struct Pop { ~Pop() { nvtx_pop(); } } pop;
+  const PopArgs a = pop_args(mode, start_ms, end_ms, n_items);
   int32_t *d_item, *d_counts;
   long long *d_t;
   unsigned long long *d_tot;
@@ -2648,6 +2694,253 @@ int cco_pop_model(cco_ctx_t *ctx, int32_t mode, int64_t n_events, const int32_t 
   CK(cudaStreamSynchronize(s));
   CK(cudaGetLastError());
   return CCO_OK;
+}
+
+// ---- URModel.save document content: correlators + rank fields + item properties (cco_model.cuh) ------------------------
+namespace cco {
+// the host-side checks of a dictionary: offsets[0] == 0, offsets[n] >= 0, bytes present; the device checks the rest
+static int check_dict_host(const cco_dictionary_t &d, const char *what, int k) {
+  if (d.n < 0 || !d.offsets) return set_error(CCO_E_INVALID_ARG, "%s %d: negative size or null offsets", what, k);
+  if (d.offsets[0] != 0) return set_error(CCO_E_INVALID_ARG, "%s %d: offsets[0] != 0", what, k);
+  if (d.offsets[d.n] < 0) return set_error(CCO_E_INVALID_ARG, "%s %d: offsets decrease", what, k);
+  if (d.offsets[d.n] > 0 && !d.bytes) return set_error(CCO_E_INVALID_ARG, "%s %d: null bytes", what, k);
+  return CCO_OK;
+}
+}  // namespace cco
+
+int cco_format_model_bulk(cco_ctx_t *ctx, const cco_result_t *res, int32_t n_names, const char *const *names,
+                          const cco_dictionary_t *row_ids, const cco_dictionary_t *col_ids, int32_t n_rankings,
+                          const cco_ranking_t *rankings, const cco_dictionary_t *prop_ids, const cco_dictionary_t *prop_json,
+                          uint32_t flags, char **out_bytes, int64_t *out_len) {
+  if (!ctx || !res || !names || !row_ids || !col_ids || !out_bytes || !out_len || n_rankings < 0 || (n_rankings > 0 && !rankings))
+    return set_error(CCO_E_INVALID_ARG, "null argument");
+  if (!prop_ids != !prop_json) return set_error(CCO_E_INVALID_ARG, "prop_ids and prop_json go together");
+  if (n_rankings > kMaxRankings) return set_error(CCO_E_UNSUPPORTED, "at most %d rankings (popular, trending, hot)", kMaxRankings);
+  CKR(check_indicators(res, n_names, names, col_ids));
+  const ResultMat &m0 = res->mats[0];
+  if (m0.row_begin != 0 || m0.row_end != m0.n_cols)
+    return set_error(CCO_E_UNSUPPORTED, "the result holds rows [%lld, %lld) of %d: format the merged model, not one rank's slice",
+                     (long long)m0.row_begin, (long long)m0.row_end, m0.n_cols);
+  const long long n_rows = m0.n_cols;
+  if (row_ids->n != n_rows) return set_error(CCO_E_INVALID_ARG, "row dictionary has %lld ids for %lld rows", (long long)row_ids->n, n_rows);
+  CKR(check_dict_host(*row_ids, "row dictionary", 0));
+  for (int i = 0; i < n_names; ++i) CKR(check_dict_host(col_ids[i], "column dictionary", i));
+  if (prop_ids) {
+    CKR(check_dict_host(*prop_ids, "property ids", 0));
+    CKR(check_dict_host(*prop_json, "property fragments", 0));
+    if (prop_ids->n != prop_json->n)
+      return set_error(CCO_E_INVALID_ARG, "%lld property ids but %lld fragments", (long long)prop_ids->n, (long long)prop_json->n);
+  }
+  const char *rank_names[kMaxRankings];
+  for (int r = 0; r < n_rankings; ++r) {
+    const cco_ranking_t &k = rankings[r];
+    if (!k.name) return set_error(CCO_E_INVALID_ARG, "ranking %d: null name", r);
+    if (!strcmp(k.name, "id")) return set_error(CCO_E_INVALID_ARG, "ranking %d: the name \"id\" is the document id", r);
+    for (int i = 0; i < n_names; ++i)
+      if (!strcmp(k.name, names[i])) return set_error(CCO_E_INVALID_ARG, "ranking %d: name \"%s\" is an indicator name", r, k.name);
+    for (int q = 0; q < r; ++q)
+      if (!strcmp(k.name, rankings[q].name)) return set_error(CCO_E_INVALID_ARG, "ranking %d: name \"%s\" repeated", r, k.name);
+    if (k.mode < CCO_POP_POPULAR || k.mode > CCO_POP_HOT) return set_error(CCO_E_INVALID_ARG, "ranking %d: mode must be CCO_POP_POPULAR, _TRENDING or _HOT", r);
+    if (k.end_ms < k.start_ms) return set_error(CCO_E_INVALID_ARG, "ranking %d: end before start (Joda Interval would throw)", r);
+    CKR(check_dict_host(k.item, "ranking", r));
+    if (k.item.n > 0 && !k.time_ms) return set_error(CCO_E_INVALID_ARG, "ranking %d: null event times", r);
+    if (k.item.n > 0x7fffffffLL) return set_error(CCO_E_UNSUPPORTED, "ranking %d: %lld events (at most 2^31 - 1)", r, (long long)k.item.n);
+    rank_names[r] = k.name;
+  }
+  // one column of every id: the rows, then every ranking's event items, then the property ids
+  std::vector<const cco_dictionary_t *> parts = {row_ids};
+  for (int r = 0; r < n_rankings; ++r) parts.push_back(&rankings[r].item);
+  if (prop_ids) parts.push_back(prop_ids);
+  std::vector<long long> first(parts.size() + 1, 0), byte0(parts.size() + 1, 0);
+  for (size_t k = 0; k < parts.size(); ++k) {
+    first[k + 1] = first[k] + parts[k]->n;
+    byte0[k + 1] = byte0[k] + parts[k]->offsets[parts[k]->n];
+  }
+  const long long n_all = first[parts.size()];
+  if (n_all >= (1LL << 32)) return set_error(CCO_E_UNSUPPORTED, "%lld ids in all (at most 2^32 - 1)", n_all);
+  const long long prop_base = prop_ids ? first[parts.size() - 1] : n_all, n_prop = prop_ids ? prop_ids->n : 0;
+
+  cco_ctx *c = ctx->members.empty() ? ctx : ctx->members[0];   // a group's merged model is formatted on its first GPU
+  CK(cudaSetDevice(c->device));
+  cudaStream_t s = c->stream;
+  nvtx_push("cco:format_model_bulk");
+  struct Pop { ~Pop() { nvtx_pop(); } } pop;
+  mail_reset(c);
+  Arena ar(s);
+  const unsigned long long N = (unsigned long long)n_all;
+
+  // offsets first: no id byte is read before every dictionary's offsets are known not to decrease
+  long long *off_all;
+  unsigned char *bytes_all;
+  int *bad;
+  CKR(ar.alloc(&off_all, N + 1));
+  CKR(ar.alloc(&bad, 1));
+  CK(cudaMemsetAsync(bad, 0x7f, sizeof(int), s));
+  for (size_t k = 0; k < parts.size(); ++k) {
+    const long long n = parts[k]->n;
+    long long *o = off_all + first[k];
+    CK(cudaMemcpyAsync(o, parts[k]->offsets, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice, s));
+    if (n > 0) {
+      k_ingest_str_check_offsets<<<grid_for(n, 256, c->sm_count), 256, 0, s>>>(n, o, (int)k, bad);
+      c->launches++;
+    }
+    if (byte0[k] != 0) {   // rebase onto the concatenated bytes (the next part's copy rewrites the shared last entry with the same value)
+      k_add_i64<<<grid_for(n + 1, 256, c->sm_count, 2), 256, 0, s>>>(n + 1, byte0[k], o);
+      c->launches++;
+    }
+  }
+  // the other dictionaries: column ids (code 100 + i) and the fragments (code 200)
+  std::vector<const cco_dictionary_t *> others;
+  for (int i = 0; i < n_names; ++i) others.push_back(&col_ids[i]);
+  if (prop_json) others.push_back(prop_json);
+  for (size_t k = 0; k < others.size(); ++k) {
+    const long long n = others[k]->n;
+    if (n == 0) continue;
+    long long *o;
+    CKR(ar.alloc(&o, n + 1));
+    CK(cudaMemcpyAsync(o, others[k]->offsets, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice, s));
+    k_ingest_str_check_offsets<<<grid_for(n, 256, c->sm_count), 256, 0, s>>>(n, o, (int)k < n_names ? 100 + (int)k : 200, bad);
+    c->launches++;
+    ar.release(o);
+  }
+  int first_bad = 0;
+  CKR(mail_fetch(c, &first_bad, bad, sizeof(int)));
+  CKR(mail_wait(c));
+  if (first_bad != 0x7f7f7f7f) {
+    if (first_bad >= 200) return set_error(CCO_E_INVALID_ARG, "property fragments: offsets decrease");
+    if (first_bad >= 100) return set_error(CCO_E_INVALID_ARG, "column dictionary %d: offsets decrease", first_bad - 100);
+    if (first_bad == 0) return set_error(CCO_E_INVALID_ARG, "row dictionary: offsets decrease");
+    if (first_bad <= n_rankings) return set_error(CCO_E_INVALID_ARG, "ranking %d: offsets decrease", first_bad - 1);
+    return set_error(CCO_E_INVALID_ARG, "property ids: offsets decrease");
+  }
+  CKR(ar.alloc(&bytes_all, std::max<long long>(byte0[parts.size()], 1)));
+  for (size_t k = 0; k < parts.size(); ++k) {
+    const long long nb = byte0[k + 1] - byte0[k];
+    if (nb > 0) CK(cudaMemcpyAsync(bytes_all + byte0[k], parts[k]->bytes, (size_t)nb, cudaMemcpyHostToDevice, s));
+  }
+  DevCol all;
+  all.n = n_all;
+  all.off = off_all;
+  all.bytes = bytes_all;
+  const StrCols cols = one_column(all);
+
+  // group equal ids; number the classes (distinct ids) in order of first appearance; rows are classes 0 .. n_rows - 1
+  uint32_t *rep, *cflag, *cpos;
+  int *dup;   // [0] a repeated row id, [1] a repeated property id
+  CKR(ar.alloc(&rep, N));
+  CKR(ar.alloc(&cflag, N + 1));
+  CKR(ar.alloc(&cpos, N + 1));
+  CKR(ar.alloc(&dup, 2));
+  CKR(group_ids(c, ar, N, cols, (flags & CCO_FLAG_INGEST_SHORT_HASH) != 0, rep));
+  CK(cudaMemsetAsync(dup, 0, 2 * sizeof(int), s));
+  CK(cudaMemsetAsync(cflag + N, 0, sizeof(uint32_t), s));
+  const int G = grid_for(n_all, 256, c->sm_count);
+  if (N > 0) {
+    k_model_class_flags<<<G, 256, 0, s>>>(N, (unsigned long long)n_rows, rep, cflag, dup);
+    c->launches++;
+  }
+  CKR(exclusive_sum_u32(c, ar, cflag, cpos, n_all + 1));
+  uint32_t n_classes = 0;
+  CKR(mail_fetch(c, &n_classes, cpos + N, 4));
+  CKR(mail_wait(c));
+  if (n_classes > 0x7fffffffu) return set_error(CCO_E_UNSUPPORTED, "%u distinct ids (at most 2^31 - 1)", n_classes);
+  uint32_t *cls_elem, *prop_of;
+  CKR(ar.alloc(&cls_elem, n_classes));
+  CKR(ar.alloc(&prop_of, n_classes));
+  CK(cudaMemsetAsync(prop_of, 0xff, sizeof(uint32_t) * std::max<size_t>(n_classes, 1), s));
+  if (N > 0) {
+    k_model_class_elem<<<G, 256, 0, s>>>(N, rep, cpos, cls_elem);
+    c->launches++;
+  }
+  if (n_prop > 0) {
+    k_model_props<<<grid_for(n_prop, 256, c->sm_count), 256, 0, s>>>(n_prop, prop_base, rep, cpos, prop_of, dup + 1);
+    c->launches++;
+  }
+  int dups[2] = {0, 0};
+  CKR(mail_fetch(c, dups, dup, 2 * sizeof(int)));
+  CKR(mail_wait(c));
+  if (dups[0]) return set_error(CCO_E_INVALID_ARG, "two equal ids in the row dictionary");
+  if (dups[1]) return set_error(CCO_E_INVALID_ARG, "two equal property ids");
+
+  // rank histograms per class: the counting of cco_pop_model over class indices, then its scoring
+  ModelArgs ma;
+  memset(&ma, 0, sizeof ma);
+  ma.n_rank = n_rankings;
+  for (int r = 0; r < n_rankings; ++r) {
+    const cco_ranking_t &k = rankings[r];
+    const PopArgs pa = pop_args(k.mode, k.start_ms, k.end_ms, (int32_t)n_classes);
+    int32_t *counts;
+    unsigned long long *tot;
+    long long *d_t;
+    double *score;
+    unsigned char *present;
+    CKR(ar.alloc(&counts, (size_t)pa.n_buckets * n_classes));
+    CKR(ar.alloc(&tot, 4));
+    CKR(ar.alloc(&d_t, std::max<long long>(k.item.n, 1)));
+    CKR(ar.alloc(&score, n_classes));
+    CKR(ar.alloc(&present, n_classes));
+    CK(cudaMemsetAsync(counts, 0, sizeof(int32_t) * std::max<size_t>((size_t)pa.n_buckets * n_classes, 1), s));
+    CK(cudaMemsetAsync(tot, 0, 32, s));
+    if (k.item.n > 0) {
+      CK(cudaMemcpyAsync(d_t, k.time_ms, sizeof(int64_t) * (size_t)k.item.n, cudaMemcpyHostToDevice, s));
+      k_rank_count<<<grid_for(k.item.n, 256, c->sm_count), 256, 0, s>>>(k.item.n, rep + first[1 + r], cpos, d_t, pa, counts, tot);
+      c->launches++;
+    }
+    if (n_classes > 0) {
+      k_pop_score<<<grid_for(n_classes, 256, c->sm_count), 256, 0, s>>>(pa, k.mode, counts, tot, score, present);
+      c->launches++;
+    }
+    ar.release(counts);
+    ar.release(d_t);
+    ma.score[r] = score;
+    ma.present[r] = present;
+  }
+  if (n_rankings > 0) CKR(escape_names(c, ar, n_rankings, rank_names, &ma.rank_names, ma.rank_name_off));
+
+  // documents: every row, then the extra classes with a present rank or a property entry, in class order
+  ma.prop_of = prop_of;
+  ma.f.n_rows = (int32_t)n_rows;
+  uint32_t *dflag, *dpos;
+  CKR(ar.alloc(&dflag, (size_t)n_classes + 1));
+  CKR(ar.alloc(&dpos, (size_t)n_classes + 1));
+  CK(cudaMemsetAsync(dflag + n_classes, 0, sizeof(uint32_t), s));
+  if (n_classes > 0) {
+    k_model_doc_flags<<<grid_for(n_classes, 256, c->sm_count), 256, 0, s>>>(ma, n_classes, dflag);
+    c->launches++;
+  }
+  CKR(exclusive_sum_u32(c, ar, dflag, dpos, (long long)n_classes + 1));
+  uint32_t n_docs = 0;
+  CKR(mail_fetch(c, &n_docs, dpos + n_classes, 4));
+  CKR(mail_wait(c));
+  uint32_t *doc_cls, *doc_src;
+  CKR(ar.alloc(&doc_cls, n_docs));
+  CKR(ar.alloc(&doc_src, n_docs));
+  if (n_classes > 0) {
+    k_model_doc_list<<<grid_for(n_classes, 256, c->sm_count), 256, 0, s>>>(n_classes, dflag, dpos, cls_elem, doc_cls, doc_src);
+    c->launches++;
+  }
+  ma.n_docs = n_docs;
+  ma.doc_cls = doc_cls;
+
+  // the document ids, gathered and escaped; the fragments verbatim; the indicators as cco_format_es_bulk has them
+  DevCol ids;
+  std::vector<void *> unused;
+  CKR(gather_dict(c, ar, cols, doc_src, n_docs, &ids, nullptr, unused));
+  CKR(escape_dict(c, ar, DevDict{ids.off, ids.bytes, ids.n}, &ma.f.row_ids));
+  const cco_dictionary_t no_props = {0, nullptr, nullptr};
+  CKR(upload_dict(c, ar, prop_json ? *prop_json : no_props, &ma.frag));
+  FormatArgs fa;
+  memset(&fa, 0, sizeof fa);
+  CKR(upload_indicators(c, ar, res, names, col_ids, &fa));
+  fa.row_ids = ma.f.row_ids;
+  ma.f = fa;
+  return assemble_docs(
+      ctx, c, ar, (long long)n_docs,
+      [&](long long *doc_len) { k_model_doc_len<<<grid_for(n_docs, 256, c->sm_count), 256, 0, s>>>(ma, doc_len); },
+      [&](const long long *doc_off, unsigned char *out) {
+        k_model_doc_write<<<grid_for((long long)n_docs * 32, 256, c->sm_count), 256, 0, s>>>(ma, doc_off, out);
+      },
+      out_bytes, out_len);
 }
 
 void cco_free(void *p) { free(p); }

@@ -72,21 +72,24 @@ struct FormatArgs {
 
 // {"index":{"_id":"  = 17 bytes ; "}}\n{"id":"  = 11 ; closing quote of the id = 1 ; per field  ,"name":[  = name + 5 and ] = 1 ;
 // per element two quotes + a comma between elements ; }\n = 2
+__device__ __forceinline__ long long indicator_fields_len(const FormatArgs &a, int r) {
+  long long len = 0;
+  for (int i = 0; i < a.n_ind; ++i) {
+    len += (a.name_off[i + 1] - a.name_off[i]) + 5 + 1;
+    const long long s = a.row_ptr[i][r], e = a.row_ptr[i][r + 1];
+    for (long long q = s; q < e; ++q) {
+      const int32_t c = a.col[i][q];
+      len += a.col_ids[i].off[c + 1] - a.col_ids[i].off[c] + 2;
+    }
+    if (e > s) len += e - s - 1;
+  }
+  return len;
+}
 __global__ void k_doc_len(const FormatArgs a, long long *__restrict__ doc_len) {
   for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < a.n_rows; r += gridDim.x * blockDim.x) {
     const long long g = a.row_id_base + r;
     const long long idl = a.row_ids.off[g + 1] - a.row_ids.off[g];
-    long long len = 17 + idl + 11 + idl + 1 + 2;
-    for (int i = 0; i < a.n_ind; ++i) {
-      len += (a.name_off[i + 1] - a.name_off[i]) + 5 + 1;
-      const long long s = a.row_ptr[i][r], e = a.row_ptr[i][r + 1];
-      for (long long q = s; q < e; ++q) {
-        const int32_t c = a.col[i][q];
-        len += a.col_ids[i].off[c + 1] - a.col_ids[i].off[c] + 2;
-      }
-      if (e > s) len += e - s - 1;
-    }
-    doc_len[r] = len;
+    doc_len[r] = 17 + idl + 11 + idl + 1 + 2 + indicator_fields_len(a, r);
   }
 }
 
@@ -95,6 +98,46 @@ __device__ __forceinline__ void warp_copy(unsigned char *dst, const unsigned cha
 }
 __device__ __forceinline__ void warp_lit(unsigned char *dst, const char *lit, int n, int lane) {
   if (lane < n) dst[lane] = (unsigned char)lit[lane];
+}
+
+// the indicator fields of row r, written by the whole warp from w on: ,"<name>":["<col>",...] per indicator
+__device__ __forceinline__ unsigned char *warp_indicator_fields(const FormatArgs &a, int r, unsigned char *w, int lane) {
+  for (int i = 0; i < a.n_ind; ++i) {
+    const int nl = a.name_off[i + 1] - a.name_off[i];
+    warp_lit(w, ",\"", 2, lane); w += 2;
+    warp_copy(w, a.names + a.name_off[i], nl, lane); w += nl;
+    warp_lit(w, "\":[", 3, lane); w += 3;
+    const long long s = a.row_ptr[i][r], e = a.row_ptr[i][r + 1];
+    // elements: the lanes first agree on every element's offset inside the array (prefix sums of 32 at a time)
+    for (long long q0 = s; q0 < e; q0 += 32) {
+      const long long q = q0 + lane;
+      long long el = 0;
+      const unsigned char *src = nullptr;
+      if (q < e) {
+        const int32_t c = a.col[i][q];
+        src = a.col_ids[i].bytes + a.col_ids[i].off[c];
+        el = a.col_ids[i].off[c + 1] - a.col_ids[i].off[c];
+      }
+      long long mine = q < e ? el + 2 + (q > s ? 1 : 0) : 0;   // leading comma from the second element on
+      long long incl = mine;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const long long v = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += v;
+      }
+      const long long total = __shfl_sync(0xffffffffu, incl, 31);
+      if (q < e) {
+        unsigned char *p = w + (incl - mine);
+        if (q > s) *p++ = ',';
+        *p++ = '"';
+        for (long long k = 0; k < el; ++k) p[k] = src[k];   // ids are short (a few to a few dozen bytes)
+        p[el] = '"';
+      }
+      w += total;
+    }
+    warp_lit(w, "]", 1, lane); w += 1;
+  }
+  return w;
 }
 
 // one warp per document: the lanes copy every byte range cooperatively; the write position advances uniformly
@@ -111,41 +154,7 @@ __global__ void k_doc_write(const FormatArgs a, const long long *__restrict__ do
     warp_lit(w, "\"}}\n{\"id\":\"", 11, lane); w += 11;
     warp_copy(w, id, idl, lane); w += idl;
     warp_lit(w, "\"", 1, lane); w += 1;
-    for (int i = 0; i < a.n_ind; ++i) {
-      const int nl = a.name_off[i + 1] - a.name_off[i];
-      warp_lit(w, ",\"", 2, lane); w += 2;
-      warp_copy(w, a.names + a.name_off[i], nl, lane); w += nl;
-      warp_lit(w, "\":[", 3, lane); w += 3;
-      const long long s = a.row_ptr[i][r], e = a.row_ptr[i][r + 1];
-      // elements: the lanes first agree on every element's offset inside the array (prefix sums of 32 at a time)
-      for (long long q0 = s; q0 < e; q0 += 32) {
-        const long long q = q0 + lane;
-        long long el = 0;
-        const unsigned char *src = nullptr;
-        if (q < e) {
-          const int32_t c = a.col[i][q];
-          src = a.col_ids[i].bytes + a.col_ids[i].off[c];
-          el = a.col_ids[i].off[c + 1] - a.col_ids[i].off[c];
-        }
-        long long mine = q < e ? el + 2 + (q > s ? 1 : 0) : 0;   // leading comma from the second element on
-        long long incl = mine;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-          const long long v = __shfl_up_sync(0xffffffffu, incl, d);
-          if (lane >= d) incl += v;
-        }
-        const long long total = __shfl_sync(0xffffffffu, incl, 31);
-        if (q < e) {
-          unsigned char *p = w + (incl - mine);
-          if (q > s) *p++ = ',';
-          *p++ = '"';
-          for (long long k = 0; k < el; ++k) p[k] = src[k];   // ids are short (a few to a few dozen bytes)
-          p[el] = '"';
-        }
-        w += total;
-      }
-      warp_lit(w, "]", 1, lane); w += 1;
-    }
+    w = warp_indicator_fields(a, r, w, lane);
     warp_lit(w, "}\n", 2, lane);
     __syncwarp();
   }

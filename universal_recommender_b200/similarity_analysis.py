@@ -220,6 +220,55 @@ class CcoContext:
         finally:
             self._L.cco_host_free(self._h, out)
 
+    @staticmethod
+    def _raw_dictionary(ids, keep: list):
+        """a `str` list or an (offsets int64[], bytes uint8[]) pair of preparator.encode_ids -> DictionaryRawT"""
+        if isinstance(ids, tuple) and len(ids) == 2 and isinstance(ids[0], np.ndarray):
+            off, data = ids
+        else:
+            from .preparator import encode_ids
+            off, data = encode_ids(list(ids))
+        off = np.ascontiguousarray(off, dtype=np.int64)
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        keep.append((off, data))
+        return N.DictionaryRawT(len(off) - 1, off.ctypes.data_as(C.POINTER(C.c_int64)), data.ctypes.data if len(data) else None)
+
+    def format_model_bulk(self, handle, names, row_ids, col_ids, rankings=(), properties=None, flags: int = 0) -> bytes:
+        """cco_format_model_bulk on a kept result: the documents URModel.save writes with recsModel "all"
+        (URAlgorithm.scala:351-367, 537-560; URModel.scala:57-102) -- format_es_bulk's rows plus one rank field per ranking in
+        which an id is present and its property fragment, and a document of its own for every other id with a rank or a
+        property entry.  rankings = [(field name, "popular" | "trending" | "hot", item ids of the ranking's events,
+        times_ms int64[], start_ms, end_ms)]; properties = {id: fragment} or (ids, fragments), a fragment being JSON object
+        members without braces.  Ids are `str` lists or encode_ids pairs."""
+        keep: list = []
+        n = len(names)
+        rd = self._raw_dictionary(row_ids, keep)
+        cds = (N.DictionaryRawT * n)(*[self._raw_dictionary(ids, keep) for ids in col_ids])
+        nm = (C.c_char_p * n)(*[x.encode("utf-8") for x in names])
+        rk = (N.RankingT * max(len(rankings), 1))()
+        for r, (name, mode, items, times, start_ms, end_ms) in enumerate(rankings):
+            code = {"popular": 0, "trending": 1, "hot": 2}[mode] if isinstance(mode, str) else int(mode)
+            d = self._raw_dictionary(items, keep)
+            t = np.ascontiguousarray(times, dtype=np.int64)
+            keep.append(t)
+            if len(t) != d.n:
+                raise N.CcoInvalidArgument(N.E_INVALID_ARG, f"ranking {name}: {d.n} item ids but {len(t)} times")
+            nb = None if name is None else name.encode("utf-8")
+            keep.append(nb)
+            rk[r] = N.RankingT(nb, code, 0, int(start_ms), int(end_ms), d, t.ctypes.data_as(C.POINTER(C.c_int64)))
+        pid = pjs = None
+        if properties is not None:
+            ids, frags = (list(properties.keys()), list(properties.values())) if isinstance(properties, dict) else properties
+            pid, pjs = self._raw_dictionary(ids, keep), self._raw_dictionary(frags, keep)
+        out, ln = C.c_void_p(), C.c_int64()
+        N.check(self._L.cco_format_model_bulk(self._h, handle, n, nm, C.byref(rd), cds, len(rankings), rk,
+                                              C.byref(pid) if pid is not None else None, C.byref(pjs) if pjs is not None else None,
+                                              flags, C.byref(out), C.byref(ln)))
+        try:
+            return C.string_at(out.value, ln.value)
+        finally:
+            self._L.cco_host_free(self._h, out)
+
     def train_csr(self, mats: Sequence[tuple[int, int, np.ndarray, np.ndarray]], params: Sequence[tuple[int, int, Optional[float]]],
                   seed: int, flags: int = 0, copy_arrays: bool = True, keep: bool = False):
         """Raw entry (cco_train): mats = [(n_rows, n_cols, row_ptr int64, col_idx int32)], params = [(m, k, minLLR|None)].
